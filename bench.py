@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU path (mz_strm_zlib over zlib 1.3)
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's outputs as .npy files
 
 Workload (config C5, `configs[4]`, the configuration the metric is quoted on): a 16 GiB synthetic enwik-style
 buffer, cut into independent 64 KiB chunks, DEFLATE level 1 + per-chunk CRC-32 + CRC fold + join (K2+K3, K1, K4).
@@ -52,7 +53,13 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-sample-mib", type=int, default=2048)
     ap.add_argument("--sub-batches", type=int, default=0, help="pieces per shard when N>1 (all-gather of piece j overlaps compression of j+1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (config c5 only; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != "c5" or args.impl != "ours"):
+        ap.error("--dump-outputs writes the outputs of config c5, --impl ours")
     if args.size_gib is None:
         args.size_gib = {"c1": 0.0625, "c2": 0.25, "c3": 4.0, "c4": 100000 * 65536 / GiB, "c5": 16.0}[args.config]
     if args.config == "c2" and "--level" not in " ".join(sys.argv):
@@ -397,6 +404,36 @@ def run_reference(args, rank, world):
 
 
 # ---- our arm ---------------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 22  # stream bytes --dump-outputs keeps over all ranks: 16 MiB as float32 plus 32 MiB of float64 positions
+
+
+def dump_outputs(out_dir, rank, world, lib, pkg, dev, nbytes, crc, stream, stream_len, crc_rows, len_rows):
+    """--dump-outputs (config c5): what a caller of the timed path receives from its last step, as DIR/<name>.npy --
+    chunk_crc32 and chunk_compressed_bytes (one row per 64 KiB chunk), totals = [input bytes, stream bytes, CRC-32 of the
+    input], and stream_sample = bytes of the joined DEFLATE stream at the sorted positions stream_sample_positions (seed 0;
+    every position when the stream is that short). float64 holds every uint32 exactly, float32 every byte. With N GPUs each
+    rank writes its own shard's arrays with the suffix _rank<r>."""
+    import numpy as np
+    import torch
+    n = nbytes // 65536
+    rows = torch.empty(2 * n, dtype=torch.int32, device=dev)
+    pkg.check(lib.mz_cuda_memcpy_d2d(rows.data_ptr(), crc_rows, 4 * n, pkg._stream_ptr()), "dump")
+    pkg.check(lib.mz_cuda_memcpy_d2d(rows.data_ptr() + 4 * n, len_rows, 4 * n, pkg._stream_ptr()), "dump")
+    rows = rows.cpu().numpy().view(np.uint32).astype(np.float64)
+    k = DUMP_SAMPLE // world
+    pos = np.arange(stream_len) if stream_len <= k else np.sort(np.random.default_rng(0).integers(0, stream_len, k))
+    joined = torch.empty(max(stream_len, 1), dtype=torch.uint8, device=dev)
+    pkg.check(lib.mz_cuda_memcpy_d2d(joined.data_ptr(), stream, stream_len, pkg._stream_ptr()), "dump")
+    sample = joined[torch.from_numpy(pos).to(dev)].cpu().numpy().astype(np.float32)
+    del joined
+    suffix = "" if world == 1 else "_rank%d" % rank
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("chunk_crc32", rows[:n]), ("chunk_compressed_bytes", rows[n:]),
+                      ("totals", np.array([nbytes, stream_len, crc], dtype=np.float64)),
+                      ("stream_sample", sample), ("stream_sample_positions", pos.astype(np.float64))):
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), arr)
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -536,11 +573,6 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     totals = piece_totals()
     comp_bytes = sum(totals)
-    # CRC of the shard = fold of the pieces' CRCs (host arithmetic); rank 0 reports its own shard's
-    crc_whole = 0
-    for j, (b, (_, nb)) in enumerate(zip(batches, subs)):
-        c = int(b.crc_out[1].item()) & 0xFFFFFFFF
-        crc_whole = c if j == 0 else lib.mz_cuda_crc32_combine(crc_whole, c, nb)
     clocks = ClockSampler(local_rank)
     clocks.start()
     kev = [[(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(NB)] for _ in range(args.steps)]
@@ -567,6 +599,19 @@ def run_ours(args, rank, world, local_rank):
         torch.cuda.synchronize()
         assert int(head[0].item()) & 6 in (0, 4), "peer region does not start with a stored/dynamic block header"
         assert 0 < int(rows[0].item()) <= 65632, "peer rows missing"
+    # CRC of the shard = fold of the pieces' CRCs (host arithmetic); rank 0 reports its own shard's, from the last timed step
+    crc_whole = 0
+    for j, (b, (_, nb)) in enumerate(zip(batches, subs)):
+        c = int(b.crc_out[1].item()) & 0xFFFFFFFF
+        crc_whole = c if j == 0 else lib.mz_cuda_crc32_combine(crc_whole, c, nb)
+    if args.dump_outputs:
+        if world == 1:
+            b = batches[0]
+            stream, stream_len, crc_rows, len_rows = b.joined.data_ptr(), piece_totals()[0], b.chunk_crc.data_ptr(), b.out_len.data_ptr()
+        else:
+            stream, stream_len = g_mine + region_off[rank], state["base"][NB]
+            crc_rows, len_rows = t_crc + 4 * c0, t_len + 4 * c0
+        dump_outputs(args.dump_outputs, rank, world, lib, pkg, dev, shard, crc_whole, stream, stream_len, crc_rows, len_rows)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

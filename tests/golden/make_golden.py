@@ -12,8 +12,12 @@ reads the committed JSON.  Two families of vectors:
    system zlib 1.3 at several levels / window_bits, for deterministic seeded inputs, plus the CRC
    returned by the reference's mz_crypt_crc32_update (mz_crypt.c:35).  Includes the boundary cases
    the survey observed (empty input, "a", "hello" gzip, level 0 stored).
+
+It also writes ``reference_outputs.json``: the reference's outputs for the larger seeded inputs of the tests that
+compare with it, pinned by CRC-32, length and SHA-256 so that those tests need no reference build.
 """
 import ctypes
+import hashlib
 import json
 import os
 import struct
@@ -86,9 +90,40 @@ def seeded_inputs():
     }
 
 
+def _digest(stream):
+    return {"size": len(stream), "sha256": hashlib.sha256(stream).hexdigest()}
+
+
+def reference_outputs(ref):
+    """What the reference's own mz_stream_zlib / mz_crypt_crc32_update return for the seeded inputs of the tests that compare
+    with it (tests/test_oracle.py, tests/test_gpu_parity.py, tests/test_gpu_configs.py). Streams are pinned by length and
+    SHA-256: the reference's writer is zlib's deflate, so the tests rebuild each stream with CPython's zlib, prove it is the
+    reference's by the digest, and then feed it to the code under test."""
+    from datagen import mixed
+    import textgen
+    out = {"oracle": [], "parity_crc": [], "c3_member": None}
+    for seed, n in ((31, 0), (32, 1), (33, 5000), (34, 200000)):
+        data = mixed(n, seed) if n else b""
+        streams = []
+        for level, wb in ((1, -15), (6, 31), (9, -15)):
+            comp = ref.zlib_compress(data, level, wb)
+            streams.append(dict(level=level, window_bits=wb, **_digest(comp)))
+        out["oracle"].append({"seed": seed, "n": n, "crc32": ref.crc32(0, data), "streams": streams})
+    for wb in (-15, 31):
+        for level in (1, 6):
+            seed = wb + level + 50
+            out["parity_crc"].append({"seed": seed, "n": 700000, "crc32": ref.crc32(0, mixed(700000, seed))})
+    n = 128 << 20
+    text = textgen.host(n, seed=7)
+    comp = ref.zlib_compress(text, level=6, window_bits=31, write_size=1 << 20)
+    out["c3_member"] = dict(text_seed=7, n=n, level=6, window_bits=31, crc32=ref.crc32(0, text), **_digest(comp))
+    return out
+
+
 def main():
     import refshim
     ref = refshim.RefLib()
+    json.dump(reference_outputs(ref), open(os.path.join(HERE, "reference_outputs.json"), "w"), indent=1)
     vec = {"foreign": corpus_entries(), "refrun": [], "crc": []}
     inputs = seeded_inputs()
     for key, data in inputs.items():

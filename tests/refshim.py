@@ -8,7 +8,10 @@ The generic mz_stream_* dispatchers of RefLib (mz_strm.c:20-130) work on ANY obj
 member is an mz_stream {vtbl, base}, so the same calls drive the reference codec and mz_strm_cuda.
 """
 import ctypes as C
+import hashlib
+import json
 import os
+import zlib
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -24,6 +27,30 @@ PROP_COMPRESS_LEVEL, PROP_COMPRESS_METHOD, PROP_COMPRESS_WINDOW = 9, 10, 11
 
 def ref_available():
     return os.path.exists(os.path.join(ROOT, "oracle/_ref/libmzref.so"))
+
+
+# -- the reference's outputs without a reference build ---------------------------------------------------------------
+# mz_strm_zlib.c is a framing layer over zlib's deflate (memLevel 8, default strategy) and inflate, the same calls
+# CPython's zlib makes. tests/golden/reference_outputs.json pins what the reference returned for the tests' seeded inputs
+# (tests/golden/make_golden.py); a stream rebuilt here is the reference's when its length and SHA-256 match.
+def reference_outputs():
+    return json.load(open(os.path.join(ROOT, "tests/golden/reference_outputs.json")))
+
+
+def zlib_stream(data, level, window_bits):
+    co = zlib.compressobj(level, zlib.DEFLATED, window_bits)
+    return co.compress(data) + co.flush()
+
+
+def is_reference_stream(stream, pinned):
+    return len(stream) == pinned["size"] and hashlib.sha256(stream).hexdigest() == pinned["sha256"]
+
+
+def zlib_read(comp, window_bits):
+    """The reference reader's decode of one stream: (bytes, compressed bytes consumed, end of stream reached)."""
+    d = zlib.decompressobj(window_bits)
+    out = d.decompress(comp) + d.flush()
+    return out, len(comp) - len(d.unused_data), d.eof
 
 
 def _sig(fn, res, args):
