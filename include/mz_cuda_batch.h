@@ -139,6 +139,20 @@ int32_t mz_cuda_wzaes_ctr(void *d_data, const uint64_t *d_off, const uint64_t *d
 int32_t mz_cuda_wzaes_hmac(const void *d_data, const uint64_t *d_off, const uint64_t *d_len, uint32_t n, const void *d_keys, uint32_t strength, void *d_mac,
                            void *stream);
 
+/* K9: PKWARE traditional encryption (APPNOTE 6.1, "ZipCrypto"; mz_strm_pkcrypt.c) of a batch of zip entries, in place: entry e is
+ * d_data[d_off[e] .. + d_len[e]), i.e. its 12-byte encryption header followed by its (compressed) bytes. `password` is a host C
+ * string (NULL: MZ_PARAM_ERROR); every entry starts from the same keys after the password, as the reference's do.
+ *   encrypt: segmented (the key stream depends on the plaintext only): every entry is cut into fixed segments and four passes
+ *            with three carry scans run over all segments of the batch, so the time follows the total bytes, not the largest
+ *            entry. Needs a device workspace of mz_cuda_pkcrypt_workspace_bytes(sum of d_len, n) bytes; the call synchronises
+ *            `stream` once, to learn the segment count (MZ_PARAM_ERROR if the workspace is too small for it).
+ *   decrypt: one thread per entry (the byte that moves the keys is the output); no workspace. The caller checks the verifier
+ *            byte(s) at the end of each decrypted header. */
+uint64_t mz_cuda_pkcrypt_workspace_bytes(uint64_t total_len, uint32_t n);
+int32_t mz_cuda_pkcrypt_encrypt(void *d_data, const uint64_t *d_off, const uint64_t *d_len, uint32_t n, const char *password, void *d_workspace,
+                                uint64_t workspace_bytes, void *stream);
+int32_t mz_cuda_pkcrypt_decrypt(void *d_data, const uint64_t *d_off, const uint64_t *d_len, uint32_t n, const char *password, void *stream);
+
 /* K4 with caller-given destinations: slot i goes to d_dst + d_offsets[i] (no scan) -- the zip archive writer interleaves the
  * entries' streams with their local headers; and n small blobs (blob i = d_blob[d_blob_off[i] .. d_blob_off[i+1])) scattered to
  * d_dst + d_dst_off[i] (the headers themselves). */

@@ -82,6 +82,18 @@ void mz_zip_cuda_trim(void);
 int32_t mz_zip_cuda_write_archive_aes(void *base_stream, const mz_cuda_zip_item *items, uint32_t count, int16_t level, uint32_t flags,
                                       const char *password, uint8_t aes_strength, mz_cuda_zip_stats *stats);
 
+/* The same archive with every entry encrypted by PKWARE traditional encryption (APPNOTE 6.1, "ZipCrypto"; scope row f4): what the
+ * reference does per entry by stacking mz_stream_pkcrypt under the codec (mz_zip.c:1733-1755, mz_strm_pkcrypt.c), and what
+ * `minizip -p` without -s, Info-ZIP `zip -e` and the Windows shell write. Each entry's stored bytes are the 12-byte encryption
+ * header (10 random bytes, then the CRC's bytes 2 and 3: the verifier of an entry without a data descriptor, mz_zip.c:192-199)
+ * followed by the DEFLATE stream, both encrypted with the keys of the password by K9 (include/mz_cuda_batch.h) on the device.
+ * Headers: flag bit 0, method 8, version needed 20 (45 with zip64), CRC kept, compressed size = stream + 12.
+ * flags may contain MZ_ZIP_CUDA_HASH_SHA256 and MZ_ZIP_CUDA_ALL_DEVICES; MZ_ZIP_CUDA_AES or a NULL password: MZ_PARAM_ERROR.
+ * PKWARE encryption is weak by today's standards (known-plaintext attacks); it is offered because it is what most readers
+ * expect. */
+int32_t mz_zip_cuda_write_archive_pkcrypt(void *base_stream, const mz_cuda_zip_item *items, uint32_t count, int16_t level, uint32_t flags,
+                                          const char *password, mz_cuda_zip_stats *stats);
+
 /* ---- batch extraction (scope row f2): the reverse direction ---------------------------------------------------
  * The reference extracts entry by entry: mz_zip_entry_read_open(raw=0) creates a mz_stream_zlib, the caller's loop
  * reads through it, mz_zip_entry_close compares the CRC (mz_zip_rw.c:818-909, mz_zip.c:2116-2128). Here the central
@@ -104,8 +116,19 @@ int32_t mz_zip_cuda_extract_all(void *zip_handle, mz_cuda_zip_entry_cb cb, void 
  * (MZ_PASSWORD_ERROR, mz_strm_wzaes.c:133-134), the HMAC-SHA1 of the ciphertext is compared with the stored authentication code
  * (MZ_CRC_ERROR, :252-254), the ciphertext is decrypted in place and decoded like any other entry. The HOST program's container
  * must be built with HAVE_WZAES (otherwise its reader refuses such entries before this code sees them). PKWARE-encrypted entries
- * return MZ_SUPPORT_ERROR; encrypted entries without a password MZ_PASSWORD_ERROR. */
+ * return MZ_SUPPORT_ERROR here (mz_zip_cuda_extract_all_encrypted reads them); encrypted entries without a password
+ * MZ_PASSWORD_ERROR. */
 int32_t mz_zip_cuda_extract_all_aes(void *zip_handle, const char *password, mz_cuda_zip_entry_cb cb, void *userdata, mz_cuda_zip_stats *stats);
+
+/* The same for archives with plain, WinZip-AES and PKWARE-encrypted entries in any mix. A PKWARE entry (flag bit 0, no AES extra
+ * field) needs a password (MZ_PASSWORD_ERROR without one) and at least its 12-byte header (MZ_FORMAT_ERROR; for STORE the stored
+ * size must be the plain size + 12). Per round every PKWARE header is decrypted and its verifier checked before any decoding --
+ * the last header byte against the entry's pk_verify, and the byte before it too when version_needed < 2, the reference's rules
+ * (mz_strm_pkcrypt.c:154-161; the reader takes pk_verify from the CRC, or from the DOS time with a data descriptor) -- a mismatch
+ * is MZ_PASSWORD_ERROR. Then K9 decrypts the stored bytes in place, one thread per entry, and the entry is decoded and checked like
+ * any other. PKWARE has no MAC: damaged ciphertext shows as MZ_DATA_ERROR or MZ_CRC_ERROR. The HOST program's container must be
+ * built with HAVE_PKCRYPT (it fills pk_verify) and, for AES entries, HAVE_WZAES. */
+int32_t mz_zip_cuda_extract_all_encrypted(void *zip_handle, const char *password, mz_cuda_zip_entry_cb cb, void *userdata, mz_cuda_zip_stats *stats);
 
 /* sizeof the mz_zip_file mirror this library was built with: the host asserts it equals sizeof(mz_zip_file) */
 uint32_t mz_zip_cuda_abi_file_info_size(void);

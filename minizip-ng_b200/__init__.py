@@ -54,11 +54,12 @@ EXPORTS = [
     "mz_cuda_deflate_slot_bound", "mz_cuda_deflate_chunks", "mz_cuda_concat", "mz_cuda_inflate_streams",
     "mz_cuda_inflate_spec_workspace_bytes", "mz_cuda_inflate_spec_round", "mz_cuda_sha256_batch",
     "mz_cuda_wzaes_derive", "mz_cuda_wzaes_ctr", "mz_cuda_wzaes_hmac",
+    "mz_cuda_pkcrypt_workspace_bytes", "mz_cuda_pkcrypt_encrypt", "mz_cuda_pkcrypt_decrypt",
     "mz_cuda_gather_region_bound", "mz_cuda_deflate_sharded", "mz_cuda_ipc_export", "mz_cuda_ipc_open", "mz_cuda_ipc_close", "mz_cuda_memcpy_peer",
     "mz_cuda_stream_wait_event", "mz_cuda_gather", "mz_cuda_scatter_blobs",
     # include/mz_zip_cuda.h
     "mz_zip_cuda_add_buffers", "mz_zip_cuda_add_buffers_ex", "mz_zip_cuda_write_archive", "mz_zip_cuda_trim", "mz_zip_cuda_write_archive_aes", "mz_zip_cuda_extract_all",
-    "mz_zip_cuda_extract_all_aes", "mz_zip_cuda_abi_file_info_size",
+    "mz_zip_cuda_extract_all_aes", "mz_zip_cuda_abi_file_info_size", "mz_zip_cuda_write_archive_pkcrypt", "mz_zip_cuda_extract_all_encrypted",
 ]
 
 
@@ -132,6 +133,9 @@ def configure(L):
     sig("mz_cuda_wzaes_derive", i32, [vp, u32, vp, u32, u32, vp, vp])
     sig("mz_cuda_wzaes_ctr", i32, [vp, vp, vp, u32, u64, vp, u32, vp])
     sig("mz_cuda_wzaes_hmac", i32, [vp, vp, vp, u32, vp, u32, vp, vp])
+    sig("mz_cuda_pkcrypt_workspace_bytes", u64, [u64, u32])
+    sig("mz_cuda_pkcrypt_encrypt", i32, [vp, vp, vp, u32, C.c_char_p, vp, u64, vp])
+    sig("mz_cuda_pkcrypt_decrypt", i32, [vp, vp, vp, u32, C.c_char_p, vp])
     sig("mz_cuda_gather_region_bound", u64, [u64])
     sig("mz_cuda_deflate_sharded", i32, [vp, i32, i32, i32, C.POINTER(u64), C.POINTER(u64), C.POINTER(u32)])
     sig("mz_cuda_ipc_export", i32, [vp, vp])

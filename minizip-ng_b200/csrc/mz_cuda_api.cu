@@ -15,6 +15,7 @@
 #include <cstdio>
 #include "inflate_kernel.cuh"
 #include "inflate_spec_kernel.cuh"
+#include "pkcrypt_kernel.cuh"
 #include "sha256_kernel.cuh"
 #include "wzaes_kernel.cuh"
 
@@ -642,6 +643,128 @@ int32_t mz_cuda_wzaes_hmac(const void *d_data, const uint64_t *d_off, const uint
     const uint32_t cap = (uint32_t)c->sm_count * 16u;
     if (blocks > cap) blocks = cap;
     MZ_LAUNCH(wzaes_hmac_kernel, dim3(blocks), dim3(128), 0, (cudaStream_t)stream, P);
+    CK(cudaGetLastError());
+    return MZ_OK;
+}
+
+/* ---- K9: PKWARE traditional encryption for a batch of entries ------------------------------------------------ */
+namespace {
+/* segment size: PK_SEG, or MZ_CUDA_PKCRYPT_SEG (a power of two, 256 .. 65536) for tuning */
+uint32_t pk_seg_size() {
+    const char *v = getenv("MZ_CUDA_PKCRYPT_SEG");
+    if (v) {
+        const long s = atol(v);
+        if (s >= 256 && s <= 65536 && (s & (s - 1)) == 0) return (uint32_t)s;
+    }
+    return PK_SEG;
+}
+/* workspace layout (all pieces 256-byte aligned): per entry the segment counts and their scan, per segment its entry, the
+ * three in-tile scans and two key starts, per tile the three aggregates, their flags and the three carries */
+uint64_t pk_layout(PkParams *P, uint8_t *w, uint64_t nseg, uint32_t n) {
+    const uint64_t tiles = (nseg + PK_THREADS - 1) / PK_THREADS;
+    uint64_t o = 0;
+    auto take = [&](uint64_t bytes) { uint8_t *p = w ? w + o : nullptr; o += al256(bytes); return p; };
+    uint8_t *seg_count = take((uint64_t)n * 4), *seg_base = take(((uint64_t)n + 1) * 8), *seg_entry = take(nseg * 4);
+    uint8_t *ks0 = take(nseg * 4), *ks1 = take(nseg * 4);
+    uint8_t *incl[3], *agg[3], *aggf[3], *pre[3];
+    for (int i = 0; i < 3; i++) {
+        incl[i] = take(nseg * 8);
+        agg[i] = take(tiles * 8);
+        aggf[i] = take(tiles * 4);
+        pre[i] = take(tiles * 8);
+    }
+    if (P) {
+        P->seg_count = (uint32_t *)seg_count;
+        P->seg_base = (const uint64_t *)seg_base;
+        P->seg_entry = (uint32_t *)seg_entry;
+        P->ks0 = (uint32_t *)ks0;
+        P->ks1 = (uint32_t *)ks1;
+        for (int i = 0; i < 3; i++) {
+            P->incl[i] = (uint2 *)incl[i];
+            P->agg[i] = (uint2 *)agg[i];
+            P->aggf[i] = (uint32_t *)aggf[i];
+            P->pre[i] = (uint2 *)pre[i];
+        }
+    }
+    return o;
+}
+} // namespace
+
+uint64_t mz_cuda_pkcrypt_workspace_bytes(uint64_t total_len, uint32_t n) {
+    return pk_layout(nullptr, nullptr, total_len / pk_seg_size() + n, n) + 256;
+}
+
+int32_t mz_cuda_pkcrypt_encrypt(void *d_data, const uint64_t *d_off, const uint64_t *d_len, uint32_t n, const char *password, void *d_workspace,
+                                uint64_t workspace_bytes, void *stream) {
+    DeviceCtx *c;
+    int32_t err = get_ctx(&c);
+    if (err) return err;
+    if (!password) return MZ_PARAM_ERROR;
+    if (n == 0) return MZ_OK;
+    if (!d_data || !d_off || !d_len || !d_workspace) return MZ_PARAM_ERROR;
+    cudaStream_t s = (cudaStream_t)stream;
+    PkParams P;
+    memset(&P, 0, sizeof(P));
+    P.data = (uint8_t *)d_data;
+    P.off = d_off;
+    P.len = d_len;
+    P.n = n;
+    P.seg = pk_seg_size();
+    uint32_t keys[3];
+    pk_host_keys(password, keys);
+    P.key0 = keys[0];
+    P.key1 = keys[1];
+    P.key2 = keys[2];
+    uint8_t *w = (uint8_t *)(((uintptr_t)d_workspace + 255) & ~(uintptr_t)255);
+    const uint64_t usable = workspace_bytes > (uint64_t)(w - (uint8_t *)d_workspace) ? workspace_bytes - (uint64_t)(w - (uint8_t *)d_workspace) : 0;
+    if (pk_layout(&P, w, 0, n) > usable) return MZ_PARAM_ERROR;
+    /* segments per entry and where each entry's segments begin; the total decides the grids and the rest of the layout */
+    const uint32_t ge = (n + 255) / 256 < (uint32_t)c->sm_count * 8u ? (n + 255) / 256 : (uint32_t)c->sm_count * 8u;
+    MZ_LAUNCH(pk_count_kernel, dim3(ge), dim3(256), 0, s, P);
+    MZ_LAUNCH(scan_lengths_kernel, dim3(1), dim3(SCAN_THREADS), 0, s, (const uint32_t *)P.seg_count, n, (uint64_t)0, (uint64_t *)P.seg_base);
+    uint64_t nseg = 0;
+    CK(cudaMemcpyAsync(&nseg, P.seg_base + n, 8, cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
+    if (nseg == 0) return MZ_OK;
+    if (nseg > 0xffffffffull - PK_THREADS || pk_layout(&P, w, nseg, n) > usable) return MZ_PARAM_ERROR; /* smaller than mz_cuda_pkcrypt_workspace_bytes */
+    P.nseg = (uint32_t)nseg;
+    P.ntiles = (uint32_t)((nseg + PK_THREADS - 1) / PK_THREADS);
+    P.xseg = gf2_xpow(g_consts.x2n, 8ull * P.seg);
+    P.aseg = 1;
+    for (uint32_t i = 0; i < P.seg; i++) P.aseg *= PK_MUL;
+    const uint32_t gt = P.ntiles < (uint32_t)c->sm_count * 6u ? P.ntiles : (uint32_t)c->sm_count * 6u;
+    MZ_LAUNCH(pk_pass1_kernel, dim3(gt), dim3(PK_THREADS), 0, s, P);
+    MZ_LAUNCH((pk_tile_scan_kernel<0, 0>), dim3(1), dim3(PK_TILE_SCAN_THREADS), 0, s, P);
+    MZ_LAUNCH(pk_pass2_kernel, dim3(gt), dim3(PK_THREADS), 0, s, P);
+    MZ_LAUNCH((pk_tile_scan_kernel<1, 1>), dim3(1), dim3(PK_TILE_SCAN_THREADS), 0, s, P);
+    MZ_LAUNCH(pk_pass3_kernel, dim3(gt), dim3(PK_THREADS), 0, s, P);
+    MZ_LAUNCH((pk_tile_scan_kernel<0, 2>), dim3(1), dim3(PK_TILE_SCAN_THREADS), 0, s, P);
+    MZ_LAUNCH(pk_pass4_kernel, dim3(gt), dim3(PK_THREADS), 0, s, P);
+    CK(cudaGetLastError());
+    return MZ_OK;
+}
+
+int32_t mz_cuda_pkcrypt_decrypt(void *d_data, const uint64_t *d_off, const uint64_t *d_len, uint32_t n, const char *password, void *stream) {
+    DeviceCtx *c;
+    int32_t err = get_ctx(&c);
+    if (err) return err;
+    if (!password) return MZ_PARAM_ERROR;
+    if (n == 0) return MZ_OK;
+    if (!d_data || !d_off || !d_len) return MZ_PARAM_ERROR;
+    PkDecParams P;
+    P.data = (uint8_t *)d_data;
+    P.off = d_off;
+    P.len = d_len;
+    P.n = n;
+    uint32_t keys[3];
+    pk_host_keys(password, keys);
+    P.key0 = keys[0];
+    P.key1 = keys[1];
+    P.key2 = keys[2];
+    uint32_t blocks = (n + PKD_THREADS - 1) / PKD_THREADS;
+    const uint32_t cap = (uint32_t)c->sm_count * 64u;
+    if (blocks > cap) blocks = cap;
+    MZ_LAUNCH(pk_decrypt_kernel, dim3(blocks), dim3(PKD_THREADS), 0, (cudaStream_t)stream, P);
     CK(cudaGetLastError());
     return MZ_OK;
 }

@@ -17,6 +17,8 @@
 #include "mz_zip_cuda.h"
 
 #define ZC_CHUNK 65536u
+/* internal flag of the native writer next to MZ_ZIP_CUDA_AES: PKWARE traditional encryption (mz_zip_cuda_write_archive_pkcrypt) */
+#define ZA_PKCRYPT 0x100u
 
 /* mz_zip.h:25-51 (mz_zip_file): the raw seam takes this struct by pointer and copies it (mz_zip.c:1939) */
 typedef struct zc_file_info_s {
@@ -410,9 +412,14 @@ typedef struct za_slot_s {
     uint32_t strength, pw_len;
     uint8_t *h_salt, *d_salt, *h_keys, *d_keys, *d_pw, *h_mac, *d_mac;
     uint64_t *h_coff, *d_coff, *h_clen, *d_clen;
+    /* PKWARE (internal flag ZA_PKCRYPT): the salt, offset and length tables above (10 random header bytes per entry, its
+     * encryption header + stream) and K9's workspace */
+    uint8_t *d_pkws;
+    uint64_t pkws_bytes;
     pthread_t th;
     int running;
     int has_aes; /* the AES buffers exist (pool matching) */
+    int has_pk;  /* the PKWARE buffers exist */
 } za_slot;
 
 static void put16(uint8_t *p, uint32_t v) { p[0] = (uint8_t)v; p[1] = (uint8_t)(v >> 8); }
@@ -462,13 +469,15 @@ static void za_free(za_slot *z) {
     mz_cuda_free(z->d_coff);
     mz_cuda_host_free(z->h_clen);
     mz_cuda_free(z->d_clen);
+    mz_cuda_free(z->d_pkws);
     free(z->meta);
     memset(z, 0, sizeof(*z));
 }
 
-static int za_alloc(za_slot *z, size_t round_bytes, uint32_t max_chunks, size_t blob_cap, int aes) {
+static int za_alloc(za_slot *z, size_t round_bytes, uint32_t max_chunks, size_t blob_cap, int aes, int pk) {
     memset(z, 0, sizeof(*z));
     z->has_aes = aes;
+    z->has_pk = pk;
     if (!zc_alloc(&z->b, round_bytes, max_chunks, 0))
         return 0;
     z->blob_cap = blob_cap;
@@ -486,20 +495,33 @@ static int za_alloc(za_slot *z, size_t round_bytes, uint32_t max_chunks, size_t 
     z->h_region = (uint8_t *)mz_cuda_host_alloc(z->region_cap);
     z->meta = (za_meta *)malloc((size_t)max_chunks * sizeof(za_meta));
     z->stream = mz_cuda_stream_create();
-    if (aes) {
+    if (aes || pk) {
         z->h_salt = (uint8_t *)mz_cuda_host_alloc((size_t)max_chunks * 16);
+        z->h_coff = (uint64_t *)mz_cuda_host_alloc((size_t)max_chunks * 8);
+        z->d_coff = (uint64_t *)mz_cuda_malloc((size_t)max_chunks * 8);
+        z->h_clen = (uint64_t *)mz_cuda_host_alloc((size_t)max_chunks * 8);
+        z->d_clen = (uint64_t *)mz_cuda_malloc((size_t)max_chunks * 8);
+        if (!z->h_salt || !z->h_coff || !z->d_coff || !z->h_clen || !z->d_clen) {
+            za_free(z);
+            return 0;
+        }
+    }
+    if (pk) { /* the encrypted ranges of a round lie inside its region, one per entry (an entry has at least one chunk) */
+        z->pkws_bytes = mz_cuda_pkcrypt_workspace_bytes(z->region_cap, max_chunks);
+        z->d_pkws = (uint8_t *)mz_cuda_malloc(z->pkws_bytes);
+        if (!z->d_pkws) {
+            za_free(z);
+            return 0;
+        }
+    }
+    if (aes) {
         z->d_salt = (uint8_t *)mz_cuda_malloc((size_t)max_chunks * 16);
         z->h_keys = (uint8_t *)mz_cuda_host_alloc((size_t)max_chunks * MZ_CUDA_WZAES_KEYREC);
         z->d_keys = (uint8_t *)mz_cuda_malloc((size_t)max_chunks * MZ_CUDA_WZAES_KEYREC);
         z->d_pw = (uint8_t *)mz_cuda_malloc(256);
         z->h_mac = (uint8_t *)mz_cuda_host_alloc((size_t)max_chunks * 20);
         z->d_mac = (uint8_t *)mz_cuda_malloc((size_t)max_chunks * 20);
-        z->h_coff = (uint64_t *)mz_cuda_host_alloc((size_t)max_chunks * 8);
-        z->d_coff = (uint64_t *)mz_cuda_malloc((size_t)max_chunks * 8);
-        z->h_clen = (uint64_t *)mz_cuda_host_alloc((size_t)max_chunks * 8);
-        z->d_clen = (uint64_t *)mz_cuda_malloc((size_t)max_chunks * 8);
-        if (!z->h_salt || !z->d_salt || !z->h_keys || !z->d_keys || !z->d_pw || !z->h_mac || !z->d_mac || !z->h_coff || !z->d_coff || !z->h_clen ||
-            !z->d_clen) {
+        if (!z->d_salt || !z->h_keys || !z->d_keys || !z->d_pw || !z->h_mac || !z->d_mac) {
             za_free(z);
             return 0;
         }
@@ -525,12 +547,13 @@ static int za_pool_enabled(void) {
     return !(v && v[0] == '0');
 }
 
-static int za_acquire(za_slot *z, int32_t dev, size_t round_bytes, uint32_t max_chunks, size_t blob_cap, int aes) {
+static int za_acquire(za_slot *z, int32_t dev, size_t round_bytes, uint32_t max_chunks, size_t blob_cap, int aes, int pk) {
     int hit = 0;
     pthread_mutex_lock(&g_za_mu);
     for (int i = 0; i < g_za_n; i++) {
         const za_slot *q = &g_za_pool[i];
-        if (q->device == dev && q->b.round_bytes >= round_bytes && q->b.max_chunks >= max_chunks && q->blob_cap >= blob_cap && (q->has_aes || !aes)) {
+        if (q->device == dev && q->b.round_bytes >= round_bytes && q->b.max_chunks >= max_chunks && q->blob_cap >= blob_cap && (q->has_aes || !aes) &&
+            (q->has_pk || !pk)) {
             *z = *q;
             g_za_pool[i] = g_za_pool[--g_za_n];
             hit = 1;
@@ -548,7 +571,7 @@ static int za_acquire(za_slot *z, int32_t dev, size_t round_bytes, uint32_t max_
         z->password = NULL;
         return 1;
     }
-    if (!za_alloc(z, round_bytes, max_chunks, blob_cap, aes))
+    if (!za_alloc(z, round_bytes, max_chunks, blob_cap, aes, pk))
         return 0;
     z->device = dev;
     return 1;
@@ -630,16 +653,20 @@ static void *za_prepare(void *arg) {
     if (!err) err = mz_cuda_memcpy_h2d(b->d_len, b->h_len, (size_t)nch * 4, z->stream);
     if (!err) err = mz_cuda_memcpy_h2d(b->d_flags, b->h_flags, nch, z->stream);
     double t1 = now_ms();
-    const int aes = (z->flags & MZ_ZIP_CUDA_AES) != 0;
+    const int aes = (z->flags & MZ_ZIP_CUDA_AES) != 0, pk = (z->flags & ZA_PKCRYPT) != 0;
     const uint32_t slen = aes ? 4 * z->strength + 4 : 0; /* MZ_AES_SALT_LENGTH */
-    if (!err && aes) { /* a fresh salt per entry (mz_strm_wzaes.c:85-86), then every entry's keys and password verifier by K8 */
+    /* bytes between an entry's local header and its stream: AES salt + verifier, or the PKWARE encryption header */
+    const uint32_t xenc = aes ? slen + 2 : (pk ? 12u : 0u);
+    if (!err && (aes || pk)) { /* fresh random bytes per entry: the AES salt (mz_strm_wzaes.c:85-86), the PKWARE header's first 10 (mz_strm_pkcrypt.c:112-113) */
         size_t got = 0;
         while (got < (size_t)ne * 16) {
             ssize_t k = getrandom(z->h_salt + got, (size_t)ne * 16 - got, 0);
             if (k <= 0) { err = MZ_INTERNAL_ERROR; break; }
             got += (size_t)k;
         }
-        if (!err) err = mz_cuda_memcpy_h2d(z->d_salt, z->h_salt, (size_t)ne * 16, z->stream);
+    }
+    if (!err && aes) { /* every entry's keys and password verifier by K8 */
+        err = mz_cuda_memcpy_h2d(z->d_salt, z->h_salt, (size_t)ne * 16, z->stream);
         if (!err) err = mz_cuda_memcpy_h2d(z->d_pw, z->password, z->pw_len ? z->pw_len : 1, z->stream);
         if (!err) err = mz_cuda_wzaes_derive(z->d_pw, z->pw_len, z->d_salt, ne, z->strength, z->d_keys, z->stream);
         if (!err) err = mz_cuda_memcpy_d2h(z->h_keys, z->d_keys, (size_t)ne * MZ_CUDA_WZAES_KEYREC, z->stream);
@@ -673,15 +700,16 @@ static void *za_prepare(void *arg) {
         const uint32_t xaes = aes ? 11u : 0u;
         const uint32_t xlen = xaes + ((z->flags & MZ_ZIP_CUDA_HASH_SHA256) ? 40u : 0u);
         const uint32_t lh = 30 + (uint32_t)nlen + xlen;
-        const uint64_t stored = csize + (aes ? slen + 2 + 10 : 0); /* salt | verifier | ciphertext | authentication code */
-        if (bo + lh + slen + 2 > z->blob_cap || stored >= 0xffffffffull) {
+        /* salt | verifier | ciphertext | authentication code, or encryption header | ciphertext */
+        const uint64_t stored = csize + (aes ? slen + 2 + 10 : (pk ? 12u : 0u));
+        if (bo + lh + xenc > z->blob_cap || stored >= 0xffffffffull) {
             err = MZ_INTERNAL_ERROR;
             break;
         }
         uint8_t *h = z->h_blob + bo;
         put32(h, 0x04034b50u);                       /* MZ_ZIP_MAGIC_LOCALHEADER */
         put16(h + 4, aes ? 51 : 20);                 /* version needed (mz_zip.c:703-725) */
-        put16(h + 6, (1u << 11) | (aes ? 1u : 0u));  /* MZ_ZIP_FLAG_UTF8 (| MZ_ZIP_FLAG_ENCRYPTED); no data descriptor: everything is known */
+        put16(h + 6, (1u << 11) | (aes || pk ? 1u : 0u)); /* MZ_ZIP_FLAG_UTF8 (| MZ_ZIP_FLAG_ENCRYPTED); no data descriptor: everything is known */
         put16(h + 8, aes ? 99 : 8);                  /* MZ_COMPRESS_METHOD_DEFLATE, or _AES with the real method in the extra field (:728-733) */
         put32(h + 10, za_dos_date(it->modified_date));
         put32(h + 14, crc);                          /* AE-1 (MZ_AES_VERSION 1) keeps the CRC (mz_zip.c:2117-2121) */
@@ -698,14 +726,22 @@ static void *za_prepare(void *arg) {
             memcpy(h + lh, z->h_salt + (size_t)e * 16, slen);
             memcpy(h + lh + slen, z->h_keys + (size_t)e * MZ_CUDA_WZAES_KEYREC + 64, 2);
         }
+        if (pk) { /* the PKWARE encryption header, still plain: 10 random bytes and the CRC's high bytes -- mz_zip_get_pk_verify for an entry
+                   * without a data descriptor (mz_zip.c:192-199); K9 encrypts it with the stream */
+            memcpy(h + lh, z->h_salt + (size_t)e * 16, 10);
+            h[lh + 10] = (uint8_t)(crc >> 16);
+            h[lh + 11] = (uint8_t)(crc >> 24);
+            z->h_coff[e] = cur + lh;
+            z->h_clen[e] = csize + 12;
+        }
         z->h_blob_off[e] = bo;
         z->h_hdr_off[e] = cur;
         z->meta[e].csize = stored;
         z->meta[e].crc = crc;
         z->meta[e].lh_rel = cur;
         z->meta[e].lh_size = lh;
-        bo += lh + (aes ? slen + 2 : 0);
-        cur += lh + (aes ? slen + 2 : 0);
+        bo += lh + xenc;
+        cur += lh + xenc;
         if (aes) {
             z->h_coff[e] = cur;
             z->h_clen[e] = csize;
@@ -730,6 +766,11 @@ static void *za_prepare(void *arg) {
     if (!err) err = mz_cuda_memcpy_h2d(z->d_blob, z->h_blob, (size_t)bo + 16, z->stream);
     if (!err) err = mz_cuda_gather(b->d_slots, b->stride, b->d_out_len, nch, z->d_dst_off, z->d_region, z->stream);
     if (!err) err = mz_cuda_scatter_blobs(z->d_blob, z->d_blob_off, z->d_hdr_off, ne, z->d_region, z->stream);
+    if (!err && pk) { /* K9: every entry's encryption header + stream becomes ciphertext in place */
+        err = mz_cuda_memcpy_h2d(z->d_coff, z->h_coff, (size_t)ne * 8, z->stream);
+        if (!err) err = mz_cuda_memcpy_h2d(z->d_clen, z->h_clen, (size_t)ne * 8, z->stream);
+        if (!err) err = mz_cuda_pkcrypt_encrypt(z->d_region, z->d_coff, z->d_clen, ne, z->password, z->d_pkws, z->pkws_bytes, z->stream);
+    }
     if (!err && aes) { /* the assembled streams become ciphertext in place; their HMACs follow them down */
         err = mz_cuda_memcpy_h2d(z->d_coff, z->h_coff, (size_t)ne * 8, z->stream);
         if (!err) err = mz_cuda_memcpy_h2d(z->d_clen, z->h_clen, (size_t)ne * 8, z->stream);
@@ -785,8 +826,23 @@ int32_t mz_zip_cuda_write_archive(void *base_stream, const mz_cuda_zip_item *ite
     return mz_zip_cuda_write_archive_aes(base_stream, items, count, level, flags, NULL, 0, stats);
 }
 
+static int32_t za_write_archive(void *base_stream, const mz_cuda_zip_item *items, uint32_t count, int16_t level, uint32_t flags,
+                                const char *password, uint8_t aes_strength, mz_cuda_zip_stats *stats);
+
 int32_t mz_zip_cuda_write_archive_aes(void *base_stream, const mz_cuda_zip_item *items, uint32_t count, int16_t level, uint32_t flags,
                                       const char *password, uint8_t aes_strength, mz_cuda_zip_stats *stats) {
+    return za_write_archive(base_stream, items, count, level, flags & ~ZA_PKCRYPT, password, aes_strength, stats);
+}
+
+int32_t mz_zip_cuda_write_archive_pkcrypt(void *base_stream, const mz_cuda_zip_item *items, uint32_t count, int16_t level, uint32_t flags,
+                                          const char *password, mz_cuda_zip_stats *stats) {
+    if ((flags & MZ_ZIP_CUDA_AES) || !password)
+        return MZ_PARAM_ERROR;
+    return za_write_archive(base_stream, items, count, level, flags | ZA_PKCRYPT, password, 0, stats);
+}
+
+static int32_t za_write_archive(void *base_stream, const mz_cuda_zip_item *items, uint32_t count, int16_t level, uint32_t flags,
+                                const char *password, uint8_t aes_strength, mz_cuda_zip_stats *stats) {
     mz_cuda_zip_stats st;
     int32_t err = MZ_OK;
     memset(&st, 0, sizeof(st));
@@ -796,7 +852,7 @@ int32_t mz_zip_cuda_write_archive_aes(void *base_stream, const mz_cuda_zip_item 
         level = 6;
     if (level < 0 || level > 9)
         return MZ_PARAM_ERROR;
-    const int aes = (flags & MZ_ZIP_CUDA_AES) != 0;
+    const int aes = (flags & MZ_ZIP_CUDA_AES) != 0, pk = (flags & ZA_PKCRYPT) != 0;
     if (aes_strength == 0)
         aes_strength = 3; /* MZ_AES_STRENGTH_256, the reference's default (mz_zip.c:2007-2009) */
     if (aes && (!password || strlen(password) > 128 || aes_strength > 3))
@@ -884,7 +940,7 @@ int32_t mz_zip_cuda_write_archive_aes(void *base_stream, const mz_cuda_zip_item 
     }
     for (uint32_t k = 0; k < nslots && err == MZ_OK; k++) {
         const int32_t dev = ndev > 1 ? (int32_t)(k % (uint32_t)ndev) : dev0;
-        if (mz_cuda_set_device(dev) != MZ_OK || !za_acquire(&slots[k], dev, round_bytes, max_chunks + 1, max_blob, aes)) {
+        if (mz_cuda_set_device(dev) != MZ_OK || !za_acquire(&slots[k], dev, round_bytes, max_chunks + 1, max_blob, aes, pk)) {
             err = MZ_MEM_ERROR;
             break;
         }
@@ -938,7 +994,7 @@ int32_t mz_zip_cuda_write_archive_aes(void *base_stream, const mz_cuda_zip_item 
             put32(h, 0x02014b50u);                   /* MZ_ZIP_MAGIC_CENTRALHEADER */
             put16(h + 4, (3u << 8) | 45u);           /* made by: MZ_HOST_SYSTEM_UNIX, 4.5 */
             put16(h + 6, aes ? 51 : (z64 ? 45 : 20));
-            put16(h + 8, (1u << 11) | (aes ? 1u : 0u));
+            put16(h + 8, (1u << 11) | (aes || pk ? 1u : 0u));
             put16(h + 10, aes ? 99 : 8);
             put32(h + 12, za_dos_date(it->modified_date));
             put32(h + 16, m->crc);
@@ -1042,6 +1098,8 @@ typedef struct zx_entry_s {
     uint16_t method;
     uint8_t has_sha;
     uint8_t aes;     /* 0, or the WinZip AES strength 1..3: the stored bytes are salt | verifier | ciphertext | authentication code */
+    uint8_t pk;      /* PKWARE traditional encryption: the stored bytes are the 12-byte encryption header | ciphertext */
+    uint16_t pk_verify, version_needed;
     uint8_t sha[32]; /* expected SHA-256 from the MZ_ZIP_EXTENSION_HASH extra field */
 } zx_entry;
 
@@ -1158,6 +1216,21 @@ static int zx_alloc(zx_bufs *b, size_t comp_cap, size_t out_cap, uint32_t max_en
     return 1;
 }
 
+/* PKWARE key schedule on the host, for the 12 header bytes of each entry (APPNOTE 6.1.5-6.1.6, mz_strm_pkcrypt.c:64-102) */
+static uint32_t zx_pk_reg(uint32_t r, uint32_t b) {
+    r ^= b & 0xffu;
+    for (int i = 0; i < 8; i++)
+        r = (r >> 1) ^ (0xedb88320u & (0u - (r & 1u)));
+    return r;
+}
+static uint32_t zx_pk_decode(uint32_t k[3], uint32_t c) {
+    const uint32_t t = k[2] | 2u, p = (c ^ ((t * (t ^ 1u)) >> 8)) & 0xffu;
+    k[0] = zx_pk_reg(k[0], p);
+    k[1] = (k[1] + (k[0] & 0xffu)) * 134775813u + 1u;
+    k[2] = zx_pk_reg(k[2], k[1] >> 24);
+    return p;
+}
+
 /* decode + checksum + deliver the entries collected in b->ent[0..n) */
 static int32_t zx_flush(zx_bufs *b, uint32_t n, size_t comp_used, size_t out_used, const char *password, mz_cuda_zip_entry_cb cb, void *userdata,
                         mz_cuda_zip_stats *st) {
@@ -1167,6 +1240,38 @@ static int32_t zx_flush(zx_bufs *b, uint32_t n, size_t comp_used, size_t out_use
     if (n == 0)
         return MZ_OK;
     err = mz_cuda_memcpy_h2d(b->d_comp, b->h_comp, comp_used + 32, NULL);
+    /* PKWARE entries (mz_strm_pkcrypt.c): every encryption header of the round is checked before anything is launched -- its
+     * decrypted last byte against the verifier, and the byte before it too for version_needed < 2 (:154-161) -- so a wrong password
+     * fails with MZ_PASSWORD_ERROR, not a decode error (except with probability 256^-n). Then K9 decrypts header + stream in place. */
+    uint32_t m = 0;
+    for (uint32_t i = 0; i < n && !err; i++) {
+        zx_entry *e = &b->ent[i];
+        if (!e->pk)
+            continue;
+        uint32_t k[3] = {305419896u, 591751049u, 878082192u}, hdr[12];
+        for (const unsigned char *q = (const unsigned char *)password; *q; q++) {
+            k[0] = zx_pk_reg(k[0], *q);
+            k[1] = (k[1] + (k[0] & 0xffu)) * 134775813u + 1u;
+            k[2] = zx_pk_reg(k[2], k[1] >> 24);
+        }
+        for (int j = 0; j < 12; j++)
+            hdr[j] = zx_pk_decode(k, b->h_comp[e->coff + j]);
+        if (hdr[11] != (e->pk_verify & 0xffu) || (e->version_needed < 2 && hdr[10] != (uint32_t)(e->pk_verify >> 8)))
+            err = MZ_PASSWORD_ERROR;
+        b->h_coff[m] = e->coff;
+        b->h_clen[m++] = e->csize;
+    }
+    if (!err && m) {
+        err = mz_cuda_memcpy_h2d(b->d_coff, b->h_coff, (size_t)m * 8, NULL);
+        if (!err) err = mz_cuda_memcpy_h2d(b->d_clen, b->h_clen, (size_t)m * 8, NULL);
+        if (!err) err = mz_cuda_pkcrypt_decrypt(b->d_comp, b->d_coff, b->d_clen, m, password, NULL);
+        if (!err) err = mz_cuda_stream_sync(NULL); /* (the tables are reused below) */
+        for (uint32_t i = 0; i < n; i++)
+            if (b->ent[i].pk) { /* from here on the entry is its compressed stream */
+                b->ent[i].coff += 12;
+                b->ent[i].csize -= 12;
+            }
+    }
     /* WinZip AES entries first (mz_strm_wzaes.c): keys from password + salt, verifier, HMAC of the ciphertext against the stored
      * authentication code, then the ciphertext becomes the compressed stream in place. One pass per strength present. */
     for (uint32_t strength = 1; strength <= 3 && !err; strength++) {
@@ -1293,7 +1398,18 @@ int32_t mz_zip_cuda_extract_all(void *zip_handle, mz_cuda_zip_entry_cb cb, void 
     return mz_zip_cuda_extract_all_aes(zip_handle, NULL, cb, userdata, stats);
 }
 
+static int32_t zx_extract(void *zip_handle, const char *password, int allow_pk, mz_cuda_zip_entry_cb cb, void *userdata, mz_cuda_zip_stats *stats);
+
 int32_t mz_zip_cuda_extract_all_aes(void *zip_handle, const char *password, mz_cuda_zip_entry_cb cb, void *userdata, mz_cuda_zip_stats *stats) {
+    return zx_extract(zip_handle, password, 0, cb, userdata, stats);
+}
+
+int32_t mz_zip_cuda_extract_all_encrypted(void *zip_handle, const char *password, mz_cuda_zip_entry_cb cb, void *userdata, mz_cuda_zip_stats *stats) {
+    return zx_extract(zip_handle, password, 1, cb, userdata, stats);
+}
+
+/* the entry walk of both: allow_pk = 0 keeps mz_zip_cuda_extract_all_aes's contract (PKWARE entries: MZ_SUPPORT_ERROR) */
+static int32_t zx_extract(void *zip_handle, const char *password, int allow_pk, mz_cuda_zip_entry_cb cb, void *userdata, mz_cuda_zip_stats *stats) {
     zx_bufs b;
     mz_cuda_zip_stats st;
     int32_t err;
@@ -1328,13 +1444,19 @@ int32_t mz_zip_cuda_extract_all_aes(void *zip_handle, const char *password, mz_c
         if (err != MZ_OK)
             break;
         const int enc = (fi->flag & 1u) != 0;
-        const uint32_t aes_over = enc ? 4u * fi->aes_strength + 4u + 12u : 0u; /* salt + verifier + authentication code */
-        if (enc && fi->aes_version && !password) {
+        const int pk = enc && !fi->aes_version && allow_pk; /* PKWARE traditional encryption */
+        /* salt + verifier + authentication code, or the PKWARE encryption header */
+        const uint32_t aes_over = pk ? 12u : (enc ? 4u * fi->aes_strength + 4u + 12u : 0u);
+        if (enc && (fi->aes_version || pk) && !password) {
             err = MZ_PASSWORD_ERROR; /* encrypted and no password given */
             break;
         }
-        if ((enc && (!fi->aes_version || fi->aes_strength < 1 || fi->aes_strength > 3 || strlen(password) > 128 ||
-                     fi->compressed_size < (int64_t)aes_over)) ||
+        if (pk && fi->compressed_size < 12) {
+            err = MZ_FORMAT_ERROR; /* shorter than its own encryption header */
+            break;
+        }
+        if ((enc && !pk && (!fi->aes_version || fi->aes_strength < 1 || fi->aes_strength > 3 || strlen(password) > 128 ||
+                            fi->compressed_size < (int64_t)aes_over)) ||
             (fi->compression_method != 0 && fi->compression_method != 8) || fi->compressed_size < 0 ||
             fi->uncompressed_size < 0 || fi->uncompressed_size > (1ll << 30) || fi->compressed_size > (1ll << 30)) {
             err = MZ_SUPPORT_ERROR; /* PKWARE-encrypted, another codec, or too large for the batch path */
@@ -1371,7 +1493,10 @@ int32_t mz_zip_cuda_extract_all_aes(void *zip_handle, const char *password, mz_c
         e->method = fi->compression_method;
         e->name_off = (uint32_t)names_used;
         e->has_sha = 0;
-        e->aes = enc ? fi->aes_strength : 0;
+        e->aes = enc && !pk ? fi->aes_strength : 0;
+        e->pk = (uint8_t)pk;
+        e->pk_verify = fi->pk_verify;
+        e->version_needed = fi->version_needed;
         /* extra fields are {id u16, size u16, data}; find MZ_ZIP_EXTENSION_HASH with algorithm SHA-256 (mz_zip_rw.c:478-510) */
         for (uint32_t xo = 0; fi->extrafield && xo + 4 <= fi->extrafield_size;) {
             const uint8_t *x = fi->extrafield + xo;
